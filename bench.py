@@ -246,7 +246,7 @@ def run_ours(args):
 
     def timed_pass(host_io):
         ins = [torch.tensor([p]).pin_memory() if host_io else torch.tensor([p], device=dev) for p in timed]
-        toks, edls, outs = 0, [], []
+        toks, edls, outs, last = 0, [], [], None
         l0 = ops.launch_count()
         r0 = model._rt.replays
         g0 = model._rt.graph_launches
@@ -257,6 +257,7 @@ def run_ours(args):
             o = model.generate(input_ids=x.to(dev, non_blocking=True) if host_io else x, **gen)
             seq = o.sequences.cpu() if host_io else o.sequences
             outs.append(seq)
+            last = o
             toks += seq.shape[1] - PROMPT_LEN
             edls += o.kwargs['edls'][1:]
         e1.record()
@@ -277,7 +278,7 @@ def run_ours(args):
         else:
             s_e, n_e = float(sum(edls)), float(len(edls))
         return dict(ms=ms, tokens=toks, mean_edl=s_e / max(n_e, 1), steps=n_e, launches=int(launches), outs=outs,
-                    per_rank_ms=per_rank)
+                    per_rank_ms=per_rank, last=last)
 
     trie = model.lookahead_cache
     snap = trie.snapshot()              # the trie after the disjoint warm-up: both timed passes start from it
@@ -290,6 +291,8 @@ def run_ours(args):
     sampler.stop_flag = True
     sampler.join(timeout=2)
     my_clk = sampler.summary()          # every rank samples its own GPU; rank 0 prints them all
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, res['last'])
     per_rank_clocks = [dict(my_clk, n_throttle_reasons=len(my_clk['reasons']))]
     if world > 1:
         t = torch.tensor([my_clk['sm_mhz'] or 0, my_clk['sm_max_mhz'] or 0, len(my_clk['reasons'])], device=dev)
@@ -344,6 +347,15 @@ def run_ours(args):
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(d, o):
+    """--dump-outputs: what generate() returned for the last request of the headline timed pass, as DIR/<name>.npy
+    (float64, exact for these integers): the token ids (prompt + generated) and the per-step draft / accepted lengths.
+    Prompts and weights are pure functions of the arguments, so two builds can be compared file by file."""
+    os.makedirs(d, exist_ok=True)
+    for name, v in (('sequences', o.sequences.cpu().numpy()), ('dls', o.kwargs['dls']), ('edls', o.kwargs['edls'])):
+        np.save(os.path.join(d, f'{name}.npy'), np.asarray(v, dtype=np.float64))
 
 
 def workload_config(args, world, peaks_src):
@@ -807,7 +819,10 @@ if __name__ == '__main__':
     ap.add_argument('--model', default='llama2-7b', choices=sorted(MODELS))
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-batched', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the last timed request\'s outputs to DIR/<name>.npy')
     a = ap.parse_args()
+    if a.dump_outputs and a.impl == 'reference':
+        ap.error('--dump-outputs writes the outputs of the GPU path (--impl ours)')
     if a.impl == 'reference':
         run_reference(a)
     else:

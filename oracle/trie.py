@@ -51,6 +51,8 @@ def lib():
         L.orc_tree_n_node.argtypes = [vp]
         L.orc_tree_n_output_node.restype = C.c_long
         L.orc_tree_n_output_node.argtypes = [vp]
+        L.orc_tree_export.restype = C.c_long
+        L.orc_tree_export.argtypes = [vp, C.c_int, C.c_long, vp, vp, vp]
         L.orc_cache_new.restype = vp
         L.orc_cache_new.argtypes = [ip, C.c_int, C.c_int, C.c_int]
         L.orc_cache_free.argtypes = [vp]
@@ -156,6 +158,15 @@ class OracleTree(object):
     @property
     def n_output_node(self):
         return lib().orc_tree_n_output_node(self._h)
+
+    def export(self, n_idx):
+        """Tree.nodes in pre-order, children in insertion order: (tokens int32 [n], parent rows int64 [n] with -1 for
+        a child of the root, counts float64 [n, 1 + n_idx] = freqs[-1], freqs[0], ..., freqs[n_idx - 1])"""
+        n = lib().orc_tree_export(self._h, n_idx, 0, None, None, None)
+        tok, par = np.zeros(n, dtype=np.int32), np.zeros(n, dtype=np.int64)
+        freq = np.zeros((n, 1 + n_idx), dtype=np.float64)
+        lib().orc_tree_export(self._h, n_idx, n, tok.ctypes.data, par.ctypes.data, freq.ctypes.data)
+        return tok, par, freq
 
 
 class OracleLookaheadCache(object):

@@ -351,6 +351,27 @@ void orc_tree_reset_input_freq(OTree *t, int idx) { if (t->root.nkid) reset_rec(
 long orc_tree_n_node(const OTree *t) { return t->n_node; }
 long orc_tree_n_output_node(const OTree *t) { return t->n_output_node; }
 
+/* Tree.nodes in pre-order, children in insertion order: row r gets the node's token, its parent's row (-1 for a child
+ * of the root) and freqs[-1], freqs[0], ..., freqs[n_idx - 1] (n_idx + 1 doubles).  Writes at most cap rows and
+ * returns the number of nodes. */
+static void export_rec(const ONode *p, long parent, int n_idx, long cap, long *row, int *tok, long *par, double *freq) {
+  for (int i = 0; i < p->nkid; ++i) {
+    const ONode *c = p->kid[i];
+    const long r = (*row)++;
+    if (r < cap) {
+      tok[r] = c->token; par[r] = parent;
+      freq[r * (n_idx + 1)] = c->fo;
+      for (int k = 0; k < n_idx; ++k) freq[r * (n_idx + 1) + 1 + k] = node_fi(c, k);
+    }
+    export_rec(c, r, n_idx, cap, row, tok, par, freq);
+  }
+}
+long orc_tree_export(const OTree *t, int n_idx, long cap, int *tok, long *par, double *freq) {
+  long row = 0;
+  export_rec(&t->root, -1, n_idx, cap, &row, tok, par, freq);
+  return row;
+}
+
 /* ------------------------------------------------------------------ LookaheadCache */
 /* LookaheadCache.__init__  lookahead_cache.py:337-347 */
 OCache *orc_cache_new(const int *eos, int n_eos, int max_node, int max_output_node) {

@@ -1,56 +1,68 @@
 # -*- coding: utf-8 -*-
-"""The premise of the pruned query walk (csrc/trie.cu tree_get), checked on the LIVE reference trie: whatever sequence
-of put / stream_put / reset_input_freqs / squeeze the reference executes, every node's counts bound its children's
-(`_put` adds along root paths, lookahead_cache.py:40-56; `_squeeze` halves top-down and pops whole subtrees, :302-310;
-`_reset_input_freq` zeroes top-down, :326-333).  Runs only where the reference checkout exists (the build container);
-the CUDA trie asserts the same on its own forests in tests/test_gpu_trie.py."""
+"""The premise of the pruned query walk (csrc/trie.cu tree_get), checked on the reference trie's forests: whatever
+sequence of put / stream_put / reset_input_freqs / squeeze the reference executes, every node's counts bound its
+children's (`_put` adds along root paths, lookahead_cache.py:40-56; `_squeeze` halves top-down and pops whole subtrees,
+:302-310; `_reset_input_freq` zeroes top-down, :326-333).  Three seeded request streams were run through the live
+reference and its whole forest hashed every 50 requests (tests/golden/gen_count_bound_golden.py); the CPU oracle
+replays the streams, must reproduce each recorded forest node for node and count for count, and the bound is checked
+on every node of those forests.  The CUDA trie asserts the same on its own forests in tests/test_gpu_trie.py."""
+import hashlib
 import os
-import sys
 
 import numpy as np
 import pytest
 
-REF = '/root/reference/lookahead'
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='the reference checkout only exists in the build container')
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'count_bound_streams.npz')
+CASES = [(1, 12, False), (2, 3000, True), (3, 40, False)]
+IDXS = 3                              # request slots: a node's counts are freqs[-1], freqs[0], freqs[1], freqs[2]
+MAX_NODE, MAX_OUTPUT_NODE = 64, 24    # tiny limits: squeezes actually happen
+PUT, STREAM_PUT, FINAL = 0, 1, 2      # op kinds of the recorded streams
 
 
-def _violations(nodes, parent_freqs, idxs):
-    bad = 0
-    for node in nodes.values():
-        if parent_freqs is not None:
-            for k in idxs:
-                if node.freqs.get(k, 0.0) > parent_freqs.get(k, 0.0):
-                    bad += 1
-        bad += _violations(node.children, node.freqs, idxs)
-    return bad
+def forest_digest(trees):
+    """sha256 of a forest given as (tree token, node tokens, parent rows, counts) per tree, trees in token order"""
+    h = hashlib.sha256()
+    for token, tok, par, freq in sorted(trees, key=lambda t: t[0]):
+        h.update(np.array([token, len(tok)], dtype=np.int64).tobytes())
+        h.update(np.asarray(tok, dtype=np.int64).tobytes())
+        h.update(np.asarray(par, dtype=np.int64).tobytes())
+        h.update(np.asarray(freq, dtype=np.float64).tobytes())
+    return h.hexdigest()
 
 
-@pytest.mark.parametrize('seed,vocab,zipf', [(1, 12, False), (2, 3000, True), (3, 40, False)])
+def _violations(par, freq):
+    """(child, slot) pairs whose count exceeds the parent's; a tree's root carries no counts, its children are exempt"""
+    kid = par >= 0
+    return int((freq[kid] > freq[par[kid]]).sum())
+
+
+@pytest.mark.parametrize('seed,vocab,zipf', CASES)
 def test_reference_counts_bound_their_children(seed, vocab, zipf):
-    sys.path.insert(0, REF)
-    try:
-        from lookahead.common.lookahead_cache import LookaheadCache
-    finally:
-        sys.path.remove(REF)
-    rng = np.random.default_rng(seed)
-
-    def toks(k):
-        if zipf:
-            return np.clip(rng.zipf(1.3, size=k), 3, vocab - 1).tolist()
-        return rng.integers(3, vocab, size=k).tolist()
-
-    c = LookaheadCache(eos_ids=[2])
-    c.max_node, c.max_output_node = 64, 24          # tiny limits: squeezes actually happen
-    checks = 0
-    for req in range(1500 if zipf else 300):
-        idx = req % 3
-        prompt = toks(int(rng.integers(4, 80)))
-        c.put(prompt[1:], branch_length=9, final=False, mode='input', idx=idx)
-        for _ in range(int(rng.integers(1, 10))):
-            c.stream_put(toks(int(rng.integers(1, 9))), branch_length=9, final=False, mode='output', idx=idx)
-        c.stream_put([], branch_length=9, final=True, mode='output', idx=idx)   # reset_input_freqs + squeeze (:403-406)
-        if req % 50 == 49:
-            for tree in c.mem.values():
-                assert _violations(tree.nodes, None, (-1, 0, 1, 2)) == 0
+    from oracle.trie import OracleLookaheadCache
+    z = np.load(GOLDEN)
+    ops, toks, digests = z[f's{seed}_ops'], z[f's{seed}_toks'], z[f's{seed}_digest']
+    c = OracleLookaheadCache(eos_ids=[2], max_node=MAX_NODE, max_output_node=MAX_OUTPUT_NODE)
+    at, req, checks = 0, 0, 0
+    for kind, n in ops.tolist():
+        ids = toks[at:at + n].tolist()
+        at += n
+        idx = req % IDXS
+        if kind == PUT:
+            c.put(ids, branch_length=9, final=False, mode='input', idx=idx)
+        else:
+            c.stream_put(ids, branch_length=9, final=kind == FINAL, mode='output', idx=idx)
+        if kind != FINAL:
+            continue
+        req += 1
+        if req % 50 == 0:
+            trees = []
+            for t in range(vocab):
+                tree = c.tree(t)
+                if tree is not None:
+                    trees.append((t, *tree.export(IDXS)))
+            assert forest_digest(trees) == digests[req // 50 - 1], f'forest after request {req} differs from the reference'
+            for _t, _tok, par, freq in trees:
+                assert _violations(par, freq) == 0
                 checks += 1
+    assert at == len(toks) and req // 50 == len(digests)
     assert checks > 20
