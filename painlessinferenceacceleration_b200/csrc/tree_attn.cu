@@ -6,8 +6,10 @@
 // The mask is never materialised: prefix keys [pad_len, P) are visible to every row, the n draft keys follow the
 // row's ancestor bit set (uint64 words, produced by the trie kernel) held in registers.
 //
-// One CTA = (KV split, head group).  A head group is one KV head's worth of rows packed into a single
-// UMMA M=128 tile: 2 query heads x 64 draft rows under GQA, 1 head otherwise (rows 64..127 idle for MHA/64).
+// One CTA = (KV split, head group).  A head group is up to two query heads of ONE KV head packed into a single
+// UMMA M=128 tile: 2 query heads x 64 draft rows under GQA, 1 head otherwise (rows 64..127 idle for MHA/64).  With an
+// odd group size G the last group of each KV head holds its single leftover head (rows 64..127 idle as for MHA), so a
+// pair never straddles two KV heads: group g -> KV head g / ceil(G/2), heads hkv*G + 2j (+1), j = g % ceil(G/2).
 // Warp roles (320 threads):  warp 0 = TMA producer (K/V tiles of 128 keys, 2-stage ring),
 //                            warp 1 = TMEM owner + single-thread tcgen05.mma issuer,
 //                            warps 2-9 = softmax / accumulate, two threads per row (TMEM lane == row; each
@@ -195,6 +197,7 @@ struct Params {
   int slot_planes;         // KV planes between consecutive slots' caches (0: shared cache)
   int plane0;              // first plane of the cache slot 0 addresses
   int layer, n_q_heads, n_kv_heads, np, mask_words, heads_per_cta, max_seq, n_split, tiles_per_cta;
+  int groups_per_kv;       // head groups per KV head: ceil(G / heads_per_cta)
   float scale_log2;
   // fused mode (pia_tree_attn_fused_fwd): RoPE + KV append happen here.  Q and the draft nodes' K / V come straight from
   // the fused projection output, the draft keys are one extra tile built in shared memory, the cache only holds [0, P)
@@ -246,8 +249,10 @@ k_tree_attn(const __grid_constant__ CUtensorMap map_k, const __grid_constant__ C
   if (n <= 0) return;      // idle slot: every CTA of its clusters takes this exit
   const long long row0 = (long long)slot * p.sl.rows_per_slot;  // first activation / mask row of the slot
   const int L = P + n;
-  const int hq0 = group * p.heads_per_cta;
-  const int hkv = hq0 / (p.n_q_heads / p.n_kv_heads);
+  const int G = p.n_q_heads / p.n_kv_heads;
+  const int hkv = group / p.groups_per_kv, jg = group % p.groups_per_kv;  // jg == 0: the KV head's first group
+  const int hq0 = hkv * G + jg * p.heads_per_cta;
+  const int heads_here = min(p.heads_per_cta, G - jg * p.heads_per_cta);  // 1 for the leftover head of an odd G
   // tiles: plain mode = the keys [0, L) of the cache; fused mode = the prefix tiles [0, P) of the cache + ONE draft tile
   // (the n draft keys, rotated and staged in shared memory by the softmax warps of the CTA that owns the last tile)
   const bool fused = p.fused != 0;
@@ -255,7 +260,7 @@ k_tree_attn(const __grid_constant__ CUtensorMap map_k, const __grid_constant__ C
   const int tiles_total = fused ? Tp + 1 : (L + BN - 1) / BN;
   // Work split decided on the device from the live length: tiles_per_cta tiles per CTA (more only when the
   // plan's split limit is reached); a single split writes the final output directly (no partials, no merge).
-  const int rows_used = p.heads_per_cta * p.np;          // 64 (MHA, 64 nodes) or 128
+  const int rows_used = heads_here * p.np;               // 64 (one head, 64 nodes) or 128
   const bool ded = (rows_used + MAX_SPLIT) * HD * 4 <= MRG_DED_ACC_BYTES;
   int ns = (tiles_total + p.tiles_per_cta - 1) / p.tiles_per_cta;
   if (ns > p.n_split) ns = p.n_split;
@@ -411,7 +416,7 @@ k_tree_attn(const __grid_constant__ CUtensorMap map_k, const __grid_constant__ C
     }
     if (!fused) {
       uint4 qv[8];  // Q row -> shared memory (UMMA K-major SWIZZLE_128B); each half loads one 64-wide d sub-tile
-      const bool have = hs < p.heads_per_cta && node < n;
+      const bool have = hs < heads_here && node < n;
       const uint4 *src = reinterpret_cast<const uint4 *>(p.q + ((row0 + node) * p.n_q_heads + hq0 + hs) * HD) + half * 8;
 #pragma unroll
       for (int ch = 0; ch < 8; ++ch) qv[ch] = have ? src[ch] : make_uint4(0, 0, 0, 0);
@@ -428,7 +433,7 @@ k_tree_attn(const __grid_constant__ CUtensorMap map_k, const __grid_constant__ C
       const uint4 *sn = reinterpret_cast<const uint4 *>(p.sin_t + (long long)pos * (HD / 2));
       const long long row_elems = (long long)(p.n_q_heads + 2 * p.n_kv_heads) * HD;
       const __nv_bfloat16 *xr = p.qkv + (row0 + node) * row_elems;
-      const bool have = hs < p.heads_per_cta && node < n;
+      const bool have = hs < heads_here && node < n;
       // All global loads of a batch are issued (read-only path: the compiler may not move plain loads across the shared
       // memory stores in between, and eight dependent load rounds of ~0.7 us each would serialise the prologue) before
       // the first value is used; four 16-byte chunks per batch bound the registers.
@@ -459,7 +464,7 @@ k_tree_attn(const __grid_constant__ CUtensorMap map_k, const __grid_constant__ C
         // per KV head also appends the rows to the cache for the steps to come (pretrained_model.py: the reference's
         // torch.cat of past and new K/V, modeling_llama.py:265-268)
         const bool key_row = hs == 0 && node < n;
-        const bool writer = (hq0 % (p.n_q_heads / p.n_kv_heads)) == 0;
+        const bool writer = jg == 0;
         const uint4 *ka = reinterpret_cast<const uint4 *>(xr + (long long)(p.n_q_heads + hkv) * HD) + half * 8;
         const uint4 *kb = reinterpret_cast<const uint4 *>(xr + (long long)(p.n_q_heads + hkv) * HD) + (half ^ 1) * 8;
         const uint4 *va = reinterpret_cast<const uint4 *>(xr + (long long)(p.n_q_heads + p.n_kv_heads + hkv) * HD) + half * 8;
@@ -661,7 +666,7 @@ k_tree_attn(const __grid_constant__ CUtensorMap map_k, const __grid_constant__ C
     }
     if (row == 0 && half == 0) DBG(10);
   } else {
-    if (ns > 1) { barrier_a(); cluster_sync_all(); }  // idle softmax warps (rows 64..127 of an MHA tile)
+    if (ns > 1) { barrier_a(); cluster_sync_all(); }  // idle softmax warps (rows 64..127 of a one-head tile)
   }
   if (ns > 1) {
     // combine this CTA's row slice: out[r][:] = sum_i acc_i 2^(m_i - M) / sum_i l_i 2^(m_i - M), all operands local
@@ -768,8 +773,13 @@ extern "C" int pia_attn_plan_create(const pia_attn_config_t *cfg, void *d_k_cach
   PIA_REQUIRE(p, "out of host memory");
   p->cfg = *cfg;
   const int G = cfg->n_q_heads / cfg->n_kv_heads;
-  p->heads_per_cta = (cfg->max_nodes == 64 && G % 2 == 0) ? 2 : 1;
-  p->n_groups = cfg->n_q_heads / p->heads_per_cta;
+  // 64-node drafts under GQA: two query heads of one KV head per CTA; an odd G leaves one single-head group per KV
+  // head.  PIA_ATTN_HEAD_PAIRS=0 keeps one head per CTA for odd G (A/B measurement of the two layouts)
+  bool pairs = G > 1;
+  const char *e = getenv("PIA_ATTN_HEAD_PAIRS");
+  if (pairs && G % 2 == 1 && e) pairs = atoi(e) != 0;
+  p->heads_per_cta = (cfg->max_nodes == 64 && pairs) ? 2 : 1;
+  p->n_groups = cfg->n_kv_heads * ((G + p->heads_per_cta - 1) / p->heads_per_cta);
   p->mask_words = cfg->max_nodes / 64;
   int n_sm = 148, dev = 0;
   cudaGetDevice(&dev);
@@ -839,6 +849,7 @@ static int attn_launch(pia_attn_plan_t *p, int layer, const void *d_q, const voi
   a.plane0 = slots->kv_first_slot * p->cfg.n_layers * p->cfg.n_kv_heads;
   a.layer = layer; a.n_q_heads = p->cfg.n_q_heads; a.n_kv_heads = p->cfg.n_kv_heads; a.np = p->cfg.max_nodes;
   a.mask_words = p->mask_words; a.heads_per_cta = p->heads_per_cta; a.max_seq = p->cfg.max_seq;
+  a.groups_per_kv = p->n_groups / p->cfg.n_kv_heads;
   // KV splits per (slot, head group): one wave of CTAs over ALL slots - a batch of requests brings its own parallelism,
   // so each cluster shrinks (8 slots x 32 head groups already cover the SMs without any split)
   int ns = p->n_split / slots->batch;

@@ -50,10 +50,13 @@ class LlamaMLP(nn.Module):
 class LlamaDecoderLayer(nn.Module):
     def __init__(self, cfg, device, dtype):
         super().__init__()
-        self.self_attn = LlamaAttention(cfg, device, dtype)
+        self.self_attn = self._make_attn(cfg, device, dtype)
         self.mlp = self._make_mlp(cfg, device, dtype)
         self.input_layernorm = LlamaRMSNorm(cfg.hidden_size, cfg.rms_norm_eps, device, dtype)
         self.post_attention_layernorm = LlamaRMSNorm(cfg.hidden_size, cfg.rms_norm_eps, device, dtype)
+
+    def _make_attn(self, cfg, device, dtype):
+        return LlamaAttention(cfg, device, dtype)
 
     def _make_mlp(self, cfg, device, dtype):
         return LlamaMLP(cfg, device, dtype)
@@ -130,7 +133,8 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         return sd
 
     def fuse(self):
-        """QKV and gate/up weights into single GEMM operands; the HF-named parameters become views of them"""
+        """QKV and gate/up weights (and q/k/v biases, where the family has them) into single GEMM operands; the
+        HF-named parameters become views of them"""
         if self._fused:
             return
         for layer in self.model.layers:
@@ -139,6 +143,11 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
             nq, nk = a.q_proj.weight.shape[0], a.k_proj.weight.shape[0]
             a.q_proj.weight.data, a.k_proj.weight.data, a.v_proj.weight.data = w[:nq], w[nq:nq + nk], w[nq + nk:]
             a.qkv_weight = w
+            a.qkv_bias = None
+            if a.q_proj.bias is not None:
+                bias = torch.cat([a.q_proj.bias.data, a.k_proj.bias.data, a.v_proj.bias.data]).contiguous()
+                a.q_proj.bias.data, a.k_proj.bias.data, a.v_proj.bias.data = bias[:nq], bias[nq:nq + nk], bias[nq + nk:]
+                a.qkv_bias = bias
             self._fuse_mlp(layer)
         self._fused = True
 
@@ -161,7 +170,7 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         """cos/sin exactly as LlamaRotaryEmbedding.forward returns them (reference :100, :111-127): fp32 angles,
         then cast to the model dtype"""
         c = self.config
-        hd = c.hidden_size // c.num_attention_heads
+        hd = self.geometry()['head_dim']
         rp = getattr(c, 'rope_parameters', None) or {}
         theta = float(getattr(c, 'rope_theta', None) or rp.get('rope_theta', 10000.0))
         scaling = getattr(c, 'rope_scaling', None) or ({k: v for k, v in rp.items() if k != 'rope_theta'} if rp else None)
@@ -212,7 +221,9 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         4-CTA cluster split-K (fp32 partials reduced through DSMEM) 3421; + o (cluster 4) 3527; + qkv (cluster 2)
         3482; everything 3740 - a k_gemm_ws launched behind the 200 KB-per-SM attention kernel cannot use its early
         weight streaming, and cuBLAS' 64x32 tiles win on the 32/96-tile projections.  Per launch (scripts/gemm_bench.py):
-        gate_up 31.5 us vs cuBLAS 34.6, lm_head 42.3 vs 46.6.  PIA_GEMM_SET overrides the set."""
+        gate_up 31.5 us vs cuBLAS 34.6, lm_head 42.3 vs 46.6.  PIA_GEMM_SET overrides the set, except that a biased qkv
+        projection (Qwen2) always stays on cuBLAS: k_gemm_ws has no bias epilogue, and adding the bias after a bf16
+        output would round twice where the reference's F.linear rounds once."""
         import os
         want = os.environ.get('PIA_GEMM_SET', 'gate_up,down').split(',')
         plans = {}
@@ -226,10 +237,11 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
             plans['gate_up_silu'] = ops.Gemm(cache[key], b.y, tiled=True).set_silu()
         elif 'gate_up' in want or 'gate_up_silu' in want:
             plans['gate_up'] = self._mk_gemm(layer.mlp.gate_up_weight, b.y)
-        if 'qkv' in want:
+        biased = layer.self_attn.qkv_bias is not None
+        if 'qkv' in want and not biased:
             plans['qkv'] = self._mk_gemm(layer.self_attn.qkv_weight, b.y)
         sk = int(os.environ.get('PIA_GEMM_SPLIT', '-4'))   # > 1: fp32 slices summed by the next rmsnorm; < -1: cluster
-        if 'qkv2' in want:
+        if 'qkv2' in want and not biased:
             plans['qkv'] = self._mk_gemm(layer.self_attn.qkv_weight, b.y, split_k=-2)
         if 'o' in want:
             plans['o'] = self._mk_gemm(layer.self_attn.o_proj.weight.data, b.attn, split_k=sk)
@@ -342,6 +354,8 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
             a = layer.self_attn
             if lp and 'qkv' in lp:
                 lp['qkv'].run(64, out=b.qkv)
+            elif a.qkv_bias is not None:   # Qwen2: cuBLASLt bias epilogue, one rounding of the fp32 xW^T + b
+                torch.addmm(a.qkv_bias, b.y, a.qkv_weight.t(), out=b.qkv)
             else:
                 torch.mm(b.y, a.qkv_weight.t(), out=b.qkv)
             if pf and lp and 'gate_up' in lp:
