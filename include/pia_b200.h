@@ -253,8 +253,25 @@ int pia_gemm_plan_set_pdl(pia_gemm_plan_t *g, int on);
 /* fused SiLU(gate) * up epilogue (modeling_llama.py:185-186): the weight must be laid out so that every 128-row tile
  * holds 64 gate rows followed by the 64 up rows of the same columns; d_out of pia_gemm_run is then [rows, N/2]. */
 int pia_gemm_plan_set_silu(pia_gemm_plan_t *g, int on);
+/* FP8 weight-only plans: the same projections (modeling_llama.py:254-256, :303, :185-186 and the Mixtral experts,
+ * mixtral/modeling_mixtral.py:668-683) with the weight stored as e4m3 plus one fp32 scale per output channel, quantised
+ * once at load time:
+ *   s[n] = max_k |W[n, k]| / 448 (1 for an all-zero row),   Wq = e4m3(W / s) round-to-nearest-even, saturating at 448,
+ *   Y[t, n] = bf16( s[n] * sum_k X[t, k] Wq[n, k]  (+ b[n]) )
+ * X is bf16; products and sums are fp32 (MMA accumulation); the bias, where given, is added in fp32 and the result is
+ * rounded to bf16 exactly once.  d_w_tiled_f8 holds Wq as [N/128][K/128] contiguous 16 KB blocks of 128 rows x 128 k
+ * (Wq.view(N/128,128,K/128,128).permute(0,2,1,3)); N % 128 == 0, K % 128 == 0.  d_scale: [N] fp32; d_bias: [N] bf16 or
+ * NULL.  d_x: [x_rows, K] bf16 with 1 <= x_rows <= 256; the plan launches 64, 128 or 256 token rows (the smallest that
+ * covers x_rows).  split_k as for pia_gemm_plan_create except stream-K (-1); fp32 slices are [splits][64|128|256][N],
+ * every slice scaled and the bias in slice 0.  SiLU*up is not available on these plans. */
+int pia_gemm_plan_create_fp8(const void *d_w_tiled_f8, const float *d_scale, const void *d_bias, int N, int K,
+                             const void *d_x, int x_rows, int split_k, pia_gemm_plan_t **out);
+/* grouped fp8 plan (MoE experts): d_w_tiled_f8 = the groups' tiled e4m3 weights back to back, d_scale [groups, N],
+ * X [x_rows, groups * K]; out[g] is [64|128|256, N] bf16, consecutive.  No bias, no K split. */
+int pia_gemm_plan_create_grouped_fp8(const void *d_w_tiled_f8, const float *d_scale, int groups, int N, int K,
+                                     const void *d_x, int x_rows, pia_gemm_plan_t **out);
 /* splits == 1: d_out is bf16 [rows_cap, N]; splits > 1: d_out is fp32 [splits][64][N] partial slices (sum them in
- * slice order, e.g. with pia_rmsnorm_partials).  rows <= 64 rows are written. */
+ * slice order, e.g. with pia_rmsnorm_partials).  rows <= 64 rows are written (rows <= x_rows for fp8 plans). */
 int pia_gemm_run(pia_gemm_plan_t *g, int rows, void *d_out, void *stream);
 
 /* ============================================================================================

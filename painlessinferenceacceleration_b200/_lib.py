@@ -84,6 +84,8 @@ SYMBOLS = {
     'pia_rmsnorm_partials': (C.c_int, [vp, C.c_int, C.c_int64, vp, vp, C.c_float, C.c_int, C.c_int, vp, vp, vp]),
     'pia_gemm_plan_create': (C.c_int, [vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.POINTER(vp)]),
     'pia_gemm_plan_create_grouped': (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, C.POINTER(vp)]),
+    'pia_gemm_plan_create_fp8': (C.c_int, [vp, vp, vp, C.c_int, C.c_int, vp, C.c_int, C.c_int, C.POINTER(vp)]),
+    'pia_gemm_plan_create_grouped_fp8': (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, C.POINTER(vp)]),
     'pia_gemm_plan_destroy': (C.c_int, [vp]),
     'pia_gemm_plan_splits': (C.c_int, [vp]),
     'pia_gemm_plan_set_pdl': (C.c_int, [vp, C.c_int]),

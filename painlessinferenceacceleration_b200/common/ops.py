@@ -40,6 +40,37 @@ def tile_weight(w):
     return t
 
 
+FP8_MAX = 448.0
+
+
+def quantize_fp8(w):
+    """weight-only e4m3 quantisation with one fp32 scale per output channel (include/pia_b200.h, DESIGN §3):
+    s[n] = max_k |W[n, k]| / 448 (1 for an all-zero row), Wq = e4m3(W / s) rounded to nearest even and saturated at
+    +-448.  w: [..., N, K] on any device -> (Wq float8_e4m3fn [..., N, K], s float32 [..., N])"""
+    wf = w.float()
+    s = wf.abs().amax(dim=-1) / FP8_MAX
+    s = torch.where(s == 0, torch.ones_like(s), s)
+    wq = (wf / s.unsqueeze(-1)).clamp_(-FP8_MAX, FP8_MAX).to(torch.float8_e4m3fn)
+    return wq, s
+
+
+def tile_weight_fp8(wq):
+    """e4m3 [N, K] (or [G, N, K]) -> [(G,) N/128, K/128, 128, 128]: one contiguous 16 KB block per (128-row tile,
+    128-wide k chunk), the TMA box of the fp8 GEMM plans"""
+    *lead, N, K = wq.shape
+    if N % 128 or K % 128:
+        raise ValueError(f'fp8 weights need N % 128 == 0 and K % 128 == 0, got [{N}, {K}]')
+    t = wq.reshape(*lead, N // 128, 128, K // 128, 128).transpose(-3, -2).contiguous()
+    t.pia_shape = (N, K)
+    return t
+
+
+def untile_weight_fp8(t):
+    """inverse of tile_weight_fp8"""
+    *lead, nt, kt, _, _ = t.shape
+    return t.transpose(-3, -2).reshape(*lead, nt * 128, kt * 128)
+
+
 def interleave_gate_up(w_gate_up):
     """[gate (I rows); up (I rows)] -> per 128-row tile: 64 gate rows then the 64 up rows of the same columns, the
     layout the fused SiLU*up epilogue of the GEMM expects"""
@@ -49,6 +80,10 @@ def interleave_gate_up(w_gate_up):
     g = w_gate_up[:inter].view(inter // 64, 64, K)
     u = w_gate_up[inter:].view(inter // 64, 64, K)
     return torch.cat([g, u], dim=1).reshape(two_i, K).contiguous()
+
+
+def _tok(rows):
+    return 64 if rows <= 64 else 128 if rows <= 128 else 256
 
 
 class Gemm(object):
@@ -86,6 +121,51 @@ class Gemm(object):
             L.check(self.lib.pia_gemm_plan_create_grouped(_p(weight), G, N, K, _p(x), x.shape[0], C.byref(self.h)))
         self.splits, self.N, self.weight, self._keep = 1, N, weight, (weight, x)
         self.out = torch.empty((G, 64, N), dtype=torch.bfloat16, device=weight.device)
+        return self
+
+    @classmethod
+    def fp8(cls, weight, scale, x, bias=None, split_k=1):
+        """fp8 weight-only plan (pia_gemm_plan_create_fp8): weight = tile_weight_fp8(Wq) [N/128, K/128, 128, 128],
+        scale fp32 [N], bias bf16 [N] or None, x bf16 [rows <= 256, K].  out: bf16 [x.shape[0], N], or fp32
+        [splits, tok, N] slices with tok = 64 / 128 / 256 (the smallest that covers x's rows)"""
+        N, K = weight.shape[-4] * 128, weight.shape[-3] * 128
+        assert weight.dim() == 4 and weight.dtype == torch.float8_e4m3fn and weight.is_contiguous()
+        assert scale.dtype == torch.float32 and scale.shape == (N,) and scale.is_contiguous()
+        assert bias is None or (bias.dtype == torch.bfloat16 and bias.shape == (N,) and bias.is_contiguous())
+        assert x.dtype == torch.bfloat16 and x.shape[1] == K and x.is_contiguous()
+        self = cls.__new__(cls)
+        self.lib = L.load()
+        self.h = L.vp()
+        with torch.cuda.device(weight.device):
+            L.check(self.lib.pia_gemm_plan_create_fp8(_p(weight), _p(scale), _p(bias), N, K, _p(x), x.shape[0],
+                                                      int(split_k), C.byref(self.h)))
+        self.splits = self.lib.pia_gemm_plan_splits(self.h)
+        self.N, self.weight, self._keep = N, weight, (weight, scale, bias, x)
+        self.tok = _tok(x.shape[0])
+        if self.splits == 1:
+            self.out = torch.empty((x.shape[0], N), dtype=torch.bfloat16, device=weight.device)
+        else:
+            self.out = torch.empty((self.splits, self.tok, N), dtype=torch.float32, device=weight.device)
+        return self
+
+    @classmethod
+    def grouped_fp8(cls, weight, scale, x):
+        """all experts in one launch (pia_gemm_plan_create_grouped_fp8): weight = tile_weight_fp8 of the stacked
+        [G, N, K] e4m3 weights ([G, N/128, K/128, 128, 128]), scale fp32 [G, N], x bf16 [rows <= 256, G * K];
+        out bf16 [G, tok, N]"""
+        G, N, K = weight.shape[0], weight.shape[1] * 128, weight.shape[2] * 128
+        assert weight.dim() == 5 and weight.dtype == torch.float8_e4m3fn and weight.is_contiguous()
+        assert scale.dtype == torch.float32 and scale.shape == (G, N) and scale.is_contiguous()
+        assert x.dtype == torch.bfloat16 and x.shape[1] == G * K and x.is_contiguous()
+        self = cls.__new__(cls)
+        self.lib = L.load()
+        self.h = L.vp()
+        with torch.cuda.device(weight.device):
+            L.check(self.lib.pia_gemm_plan_create_grouped_fp8(_p(weight), _p(scale), G, N, K, _p(x), x.shape[0],
+                                                              C.byref(self.h)))
+        self.splits, self.N, self.weight, self._keep = 1, N, weight, (weight, scale, x)
+        self.tok = _tok(x.shape[0])
+        self.out = torch.empty((G, self.tok, N), dtype=torch.bfloat16, device=weight.device)
         return self
 
     def set_pdl(self, on=True):

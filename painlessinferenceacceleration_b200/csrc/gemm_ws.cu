@@ -124,21 +124,64 @@ struct Params {
   int no_pdl;               // 1: plain kernel boundary - do not let the successor start early either
   __nv_bfloat16 *out_bf16;  // [rows_cap, N]  (or [rows_cap, N/2] with silu)   (n_split == 1)
   float *out_f32;           // [n_split, TOK, N] slices  (n_split > 1)
+  // fp8-weight plans only
+  const float *scale;             // [groups, N] per-output-channel dequantisation scales
+  const __nv_bfloat16 *bias;      // [N] or nullptr
+  int w_group_tiles;              // 128-row weight tiles per group (tiled fp8 blocks are [groups][tiles][chunks])
 };
+
+// ------------------------------------------------------------------------------------------------ fp8 weights
+// FP8 = true: W is e4m3 with one fp32 scale per output channel, Y[t, n] = bf16(s[n] * sum_k X[t, k] Wq[n, k] (+ b[n])).
+// A stage is one 128 x 128 e4m3 box (16 KB: half the bytes of the bf16 stage's 128 x 64) plus the two 64-k activation
+// boxes of the same 128 k.  tcgen05.mma kind::f16 needs bf16 operands, so the four epilogue warps - idle until the
+// accumulator is complete - dequantise each weight half-tile (thread = weight row) into a SWIZZLE_128B K-major bf16
+// half-tile in shared memory (two slots, recycled by tcgen05.commit), fence the generic->async proxy and hand it to
+// the MMA warp, which runs exactly the bf16 kernel's UMMA sequence on it.  The conversion is exact (every e4m3 value is
+// a bf16 value), so with the scale applied in the epilogue the only roundings are the fp32 MMA accumulation and the
+// final bf16 store.  Chosen over writing the bf16 tile to TMEM (tcgen05.st + TS-form MMA): the shared-memory form keeps
+// the MMA descriptors, the accumulator and the split-K / cluster code of the bf16 path unchanged, and the swizzled
+// layout makes the row-per-thread loads and stores bank-conflict free.
+// Activations stay bf16 on purpose: at <= 256 token rows the GEMM is bound by HBM bytes, not by the MMA rate, so
+// quantising X to e4m3 for kind::f8f6f4 would change the numerics (W8A8) for no gain in time.
+// TOKN (the UMMA N = token rows per launch) is 64 (decode, decoding_length <= 64), 128 (decode up to 128 nodes) or
+// 256 (prefill passes); shared memory per TOKN is sized so that TOKN = 64 keeps two CTAs per SM.
+constexpr int F8_BK = 128;                 // k per fp8 stage (one 128-byte swizzle row of e4m3)
+constexpr int F8_W = BMW * F8_BK;          // 16 KB e4m3 weight box
+constexpr int F8_CONV = BMW * BK * 2;      // one bf16 half tile (128 rows x 64 k)
+constexpr int f8_stage(int tokn) { return F8_W + 2 * tokn * BK * 2; }
+constexpr int f8_smem_total(int nstage, int tokn) { return nstage * f8_stage(tokn) + 2 * F8_CONV + 256 + 1024; }
+constexpr uint32_t idesc_tok(int tokn) {
+  return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(tokn >> 3) << 17) | ((uint32_t)(BMW >> 4) << 24);
+}
+__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
+  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+}
+// two e4m3 bytes at bits 15:8 and 31:24 of t -> bf16x2, exactly: sign and the 7 exponent/mantissa bits move into a
+// bf16 with exponent bias 127 instead of 7, and the multiply by 2^120 rebiases (bf16 keeps e4m3's subnormals, the
+// product is exact and -0 keeps the sign of zero)
+__device__ __forceinline__ uint32_t e4m3x2_to_bf16x2(uint32_t t) {
+  const uint32_t v = (t & 0x80008000u) | ((t >> 4) & 0x07F007F0u);
+  uint32_t r;
+  asm("fma.rn.bf16x2 %0, %1, %2, %3;" : "=r"(r) : "r"(v), "r"(0x7B807B80u), "r"(0x80008000u));
+  return r;
+}
 
 // NSTAGE = 4: ~100 KB of shared memory, two CTAs per SM (grids with more CTAs than SMs);
 // NSTAGE = 8: ~200 KB, one CTA per SM with twice the bytes in flight (grids that do not fill the SMs twice) -
 // HBM only saturates with >= ~10 MB of loads in flight chip-wide.
-template <int NSTAGE>
-__global__ void __launch_bounds__(NTHREADS, NSTAGE <= 4 ? 2 : 1)
+// FP8: NSTAGE = 2 at TOKN = 64 (~97 KB, two CTAs per SM), otherwise one CTA per SM (see f8_smem_total).
+template <int NSTAGE, int TOKN = TOK, bool FP8 = false>
+__global__ void __launch_bounds__(NTHREADS, (FP8 ? (TOKN == 64 && NSTAGE <= 2) : NSTAGE <= 4) ? 2 : 1)
 k_gemm_ws(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUtensorMap map_x, Params p) {
-  constexpr int SMEM_BAR = NSTAGE * STAGE_BYTES;
+  constexpr int SMEM_BAR = FP8 ? NSTAGE * f8_stage(TOKN) + 2 * F8_CONV : NSTAGE * STAGE_BYTES;
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t *sm = smem_raw + (base - smem_u32(smem_raw));
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const uint32_t bar_full = base + SMEM_BAR, bar_empty = bar_full + 8 * NSTAGE, bar_acc = bar_empty + 8 * NSTAGE;
-  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(sm + SMEM_BAR + 16 * NSTAGE + 16);
+  const uint32_t conv_full = bar_acc + 8, conv_empty = conv_full + 16;  // fp8: the two bf16 half-tile slots
+  uint32_t *tmem_slot = reinterpret_cast<uint32_t *>(sm + SMEM_BAR + 16 * NSTAGE + (FP8 ? 48 : 16));
+  constexpr int TMEM_N = FP8 ? TOKN : TMEM_COLS;
   // grid = (tiles, splits), or (splits, tiles) when the splits of a tile form a cluster (clusters run along x)
   const int tile = p.cluster ? blockIdx.y : blockIdx.x, split = p.cluster ? blockIdx.x : blockIdx.y;
   const int n0 = tile * BMW;
@@ -152,11 +195,14 @@ k_gemm_ws(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUt
   if (tid == 0) {
     for (int s = 0; s < NSTAGE; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
     mbar_init(bar_acc, 1);
+    if constexpr (FP8) {
+      for (int h = 0; h < 2; ++h) { mbar_init(conv_full + 8 * h, 128); mbar_init(conv_empty + 8 * h, 1); }
+    }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
   __syncwarp();  // warp 0 reconverges before the block barrier below
   if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_COLS));
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_slot)), "n"(TMEM_N));
     asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
   }
   if (!p.no_pdl) pdl_launch_dependents();
@@ -168,6 +214,157 @@ k_gemm_ws(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUt
   // NSTAGE weight tiles are already streaming from HBM before griddepcontrol.wait: only the activation tiles (and
   // the output stores) depend on the predecessor, so its run time hides this kernel's pipeline fill.
 
+  if constexpr (FP8) {
+    constexpr int XH = TOKN * BK * 2, STG = f8_stage(TOKN), CONV0 = NSTAGE * STG, QT = TOKN / 4;
+    constexpr uint32_t IDESC8 = idesc_tok(TOKN);
+    if (warp == 0) {
+      if (lane == 0) {
+        const int blk0 = (grp * p.w_group_tiles + tile) * p.n_chunks + c0;
+        auto load_x = [&](int i, int s) {  // the two 64-k activation boxes of fp8 chunk c0 + i
+          const uint32_t xd = base + s * STG + F8_W;
+          const int kc = xk0 + 2 * (c0 + i);
+          tma_load_2d(xd, &map_x, bar_full + 8 * s, kc * BK, 0);
+          tma_load_2d(xd + XH, &map_x, bar_full + 8 * s, (kc + 1) * BK, 0);
+        };
+        const int pre = nch < NSTAGE ? nch : NSTAGE;
+        for (int i = 0; i < pre; ++i) {
+          mbar_expect_tx(bar_full + 8 * i, STG);
+          tma_load_3d(base + i * STG, &map_w, bar_full + 8 * i, 0, 0, blk0 + i);
+        }
+        pdl_wait();
+        for (int i = 0; i < pre; ++i) load_x(i, i);
+        for (int i = pre; i < nch; ++i) {
+          const int s = i % NSTAGE, ph = (i / NSTAGE) & 1;
+          mbar_wait(bar_empty + 8 * s, ph ^ 1);
+          mbar_expect_tx(bar_full + 8 * s, STG);
+          tma_load_3d(base + s * STG, &map_w, bar_full + 8 * s, 0, 0, blk0 + i);
+          load_x(i, s);
+        }
+      }
+      __syncwarp();
+      if (p.cluster) { cluster_sync_all(); cluster_sync_all(); }
+    } else if (warp == 1) {
+      if (lane == 0) {
+        for (int i = 0; i < nch; ++i) {
+          const int s = i % NSTAGE, ph = (i / NSTAGE) & 1;
+          mbar_wait(bar_full + 8 * s, ph);  // activation boxes landed
+#pragma unroll
+          for (int h = 0; h < 2; ++h) {
+            mbar_wait(conv_full + 8 * h, i & 1);  // bf16 half tile h written and fenced
+            tc_fence_after();
+            const uint32_t wa = base + CONV0 + h * F8_CONV, xa = base + s * STG + F8_W + h * XH;
+#pragma unroll
+            for (int j = 0; j < BK / 16; ++j)
+              umma_bf16(tmem, kmajor_desc(wa + j * 32), kmajor_desc(xa + j * 32), IDESC8, (i | h | j) != 0);
+            umma_commit(conv_empty + 8 * h);
+          }
+          umma_commit(bar_empty + 8 * s);
+        }
+        umma_commit(bar_acc);
+      }
+      __syncwarp();
+      if (p.cluster) { cluster_sync_all(); cluster_sync_all(); }
+    } else {
+      const int q = warp & 3;
+      const int r = q * 32 + lane, r7 = r & 7;
+      // dequantise: thread = weight row r; 16-byte chunk c of a swizzled 128-byte row sits at chunk c ^ (r & 7)
+      for (int i = 0; i < nch; ++i) {
+        const int s = i % NSTAGE, ph = (i / NSTAGE) & 1;
+        mbar_wait(bar_full + 8 * s, ph);
+        const uint8_t *src = sm + s * STG + r * 128;
+#pragma unroll
+        for (int h = 0; h < 2; ++h) {
+          mbar_wait(conv_empty + 8 * h, (i & 1) ^ 1);
+          uint8_t *dst = sm + CONV0 + h * F8_CONV + r * 128;
+#pragma unroll
+          for (int c4 = 0; c4 < 4; ++c4) {
+            const uint4 f = *reinterpret_cast<const uint4 *>(src + (((h * 4 + c4) ^ r7) << 4));
+            uint4 lo, hi;
+            lo.x = e4m3x2_to_bf16x2(__byte_perm(f.x, 0, 0x1404)); lo.y = e4m3x2_to_bf16x2(__byte_perm(f.x, 0, 0x3424));
+            lo.z = e4m3x2_to_bf16x2(__byte_perm(f.y, 0, 0x1404)); lo.w = e4m3x2_to_bf16x2(__byte_perm(f.y, 0, 0x3424));
+            hi.x = e4m3x2_to_bf16x2(__byte_perm(f.z, 0, 0x1404)); hi.y = e4m3x2_to_bf16x2(__byte_perm(f.z, 0, 0x3424));
+            hi.z = e4m3x2_to_bf16x2(__byte_perm(f.w, 0, 0x1404)); hi.w = e4m3x2_to_bf16x2(__byte_perm(f.w, 0, 0x3424));
+            *reinterpret_cast<uint4 *>(dst + (((2 * c4) ^ r7) << 4)) = lo;
+            *reinterpret_cast<uint4 *>(dst + (((2 * c4 + 1) ^ r7) << 4)) = hi;
+          }
+          asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+          mbar_arrive(conv_full + 8 * h);
+        }
+      }
+      // epilogue: scale per weight row (= TMEM lane), bias, one rounding; 32 token columns at a time
+      pdl_wait();
+      if (nch > 0) { mbar_wait(bar_acc, 0); tc_fence_after(); }
+      const uint32_t a = tmem + ((uint32_t)(q * 32) << 16);
+      const float *scale = p.scale + (long long)grp * p.N;
+      uint32_t v[32];
+      auto load32 = [&](int cc) {
+        if (nch > 0) { tmem_ld32(a + cc * 32, v); tmem_ld_wait(); }
+        else {
+#pragma unroll
+          for (int t = 0; t < 32; ++t) v[t] = 0u;
+        }
+      };
+      if (p.cluster) {
+        // as the bf16 path: fp32 rows pushed to the owner CTA's (dead) stage ring, summed there in split order, then
+        // scaled, biased and rounded once
+        const int cs = p.cluster, RS = BMW / cs;
+        cluster_sync_all();
+        {
+          const int owner = r / RS, rl = r % RS;
+          const uint32_t dst = map_to_cta(base + (uint32_t)((split * QT) * RS + rl) * 16, owner);
+          for (int cc = 0; cc < TOKN / 32; ++cc) {
+            load32(cc);
+#pragma unroll
+            for (int u = 0; u < 8; ++u)
+              st_cluster_f4(dst + (uint32_t)((cc * 8 + u) * RS) * 16, __uint_as_float(v[4 * u]), __uint_as_float(v[4 * u + 1]),
+                            __uint_as_float(v[4 * u + 2]), __uint_as_float(v[4 * u + 3]));
+          }
+        }
+        cluster_sync_all();
+        {
+          const int e = (warp - 2) * 32 + lane;
+          const int rl = e % RS, tg = e / RS;
+          const int qpt = QT * RS / BMW;               // token quads per thread
+          const int n_out = n0 + split * RS + rl;
+          const float4 *buf = reinterpret_cast<const float4 *>(sm);
+          __nv_bfloat16 *ob = p.out_bf16 + grp * p.out_group_stride;
+          const float sc = scale[n_out], bb = p.bias ? __bfloat162float(p.bias[n_out]) : 0.f;
+          for (int tq = tg * qpt; tq < (tg + 1) * qpt; ++tq) {
+            float4 acc = buf[tq * RS + rl];
+            for (int src = 1; src < cs; ++src) {
+              const float4 b = buf[(src * QT + tq) * RS + rl];
+              acc.x += b.x; acc.y += b.y; acc.z += b.z; acc.w += b.w;
+            }
+            const int t0 = 4 * tq;
+            if (t0 < p.rows) ob[(long long)t0 * p.N + n_out] = __float2bfloat16_rn(sc * acc.x + bb);
+            if (t0 + 1 < p.rows) ob[(long long)(t0 + 1) * p.N + n_out] = __float2bfloat16_rn(sc * acc.y + bb);
+            if (t0 + 2 < p.rows) ob[(long long)(t0 + 2) * p.N + n_out] = __float2bfloat16_rn(sc * acc.z + bb);
+            if (t0 + 3 < p.rows) ob[(long long)(t0 + 3) * p.N + n_out] = __float2bfloat16_rn(sc * acc.w + bb);
+          }
+        }
+      } else {
+        const int n = n0 + r;  // N % 128 == 0: every row is in range
+        const float sc = scale[n];
+        // fp32 slices: every slice is scaled, the bias goes into slice 0 only
+        const float bb = (p.bias && split == 0) ? __bfloat162float(p.bias[n]) : 0.f;
+        for (int cc = 0; cc < TOKN / 32; ++cc) {
+          load32(cc);
+          if (p.n_split == 1) {
+            __nv_bfloat16 *o = p.out_bf16 + grp * p.out_group_stride + n;
+#pragma unroll
+            for (int t = 0; t < 32; ++t)
+              if (cc * 32 + t < p.rows) o[(long long)(cc * 32 + t) * p.N] = __float2bfloat16_rn(sc * __uint_as_float(v[t]) + bb);
+          } else {
+            float *o = p.out_f32 + (long long)split * TOKN * p.N + n;
+#pragma unroll
+            for (int t = 0; t < 32; ++t)
+              if (cc * 32 + t < p.rows) o[(long long)(cc * 32 + t) * p.N] = sc * __uint_as_float(v[t]) + bb;
+          }
+        }
+      }
+      tc_fence_before();
+    }
+  } else
   if (warp == 0) {
     if (lane == 0) {
       auto load_w = [&](int i, int s) {
@@ -314,7 +511,7 @@ k_gemm_ws(const __grid_constant__ CUtensorMap map_w, const __grid_constant__ CUt
   __syncthreads();
   if (warp == 1) {
     tc_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(TMEM_COLS));
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "n"(TMEM_N));
   }
 }
 
@@ -509,6 +706,7 @@ struct pia_gemm_plan {
   // stream-K mode
   int stream_k, sk_grid;
   SkParams sk;
+  int fp8, tok, x_rows;  // fp8-weight plan: token rows per launch (UMMA N) and rows of the activation buffer
 };
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
@@ -644,7 +842,7 @@ extern "C" int pia_gemm_plan_set_pdl(pia_gemm_plan_t *g, int on) {
 }
 extern "C" int pia_gemm_plan_splits(const pia_gemm_plan_t *g) { return g ? (g->p.cluster ? 1 : g->p.n_split) : 0; }
 extern "C" int pia_gemm_plan_set_silu(pia_gemm_plan_t *g, int on) {
-  PIA_REQUIRE(g && g->p.n_split == 1 && !g->stream_k && g->p.N % BMW == 0, "the SiLU*up epilogue needs split_k == 1 and N %% 128 == 0");
+  PIA_REQUIRE(g && !g->fp8 && g->p.n_split == 1 && !g->stream_k && g->p.N % BMW == 0, "the SiLU*up epilogue needs split_k == 1 and N %% 128 == 0");
   g->p.silu = on ? 1 : 0;
   return PIA_OK;
 }
@@ -681,10 +879,113 @@ extern "C" int pia_gemm_plan_create_grouped(const void *d_w, int groups, int N, 
   return PIA_OK;
 }
 
+// e4m3 weights pre-tiled by tile_weight_fp8: [blocks] contiguous 16 KB boxes of 128 rows x 128 k bytes
+static int encode_tiled_w_fp8(CUtensorMap *m, const void *base, uint64_t n_blocks) {
+  EncodeTiledFn fn = get_encode();
+  PIA_REQUIRE(fn, "cuTensorMapEncodeTiled not available in this driver");
+  cuuint64_t dims[3] = {(cuuint64_t)F8_BK, (cuuint64_t)BMW, n_blocks};
+  cuuint64_t strides[2] = {(cuuint64_t)F8_BK, (cuuint64_t)F8_BK * BMW};
+  cuuint32_t box[3] = {F8_BK, BMW, 1};
+  cuuint32_t estr[3] = {1, 1, 1};
+  CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void *>(base), dims, strides, box, estr,
+                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                  CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d", (int)r); return PIA_ERR_CUDA; }
+  return PIA_OK;
+}
+
+// the fp8 instantiations: (stages, token rows)
+template <int NS, int T>
+static cudaError_t f8_attr() {
+  return cudaFuncSetAttribute(k_gemm_ws<NS, T, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, f8_smem_total(NS, T));
+}
+template <int NS, int T>
+static cudaError_t f8_launch(const pia_gemm_plan *g, const Params &p, cudaStream_t st) {
+  const int smem = f8_smem_total(NS, T);
+  if (p.cluster)
+    return launch_kernel_cluster(k_gemm_ws<NS, T, true>, dim3(p.n_split, p.N / BMW), dim3(NTHREADS), smem, st,
+                                 (unsigned)p.cluster, g->map_w, g->map_x, p);
+  return launch_kernel(k_gemm_ws<NS, T, true>, dim3(p.N / BMW, p.n_split, p.groups), dim3(NTHREADS), smem, st, g->map_w,
+                       g->map_x, p);
+}
+
+static int fp8_plan_create(const void *d_w, const float *d_scale, const void *d_bias, int groups, int N, int K,
+                           const void *d_x, int x_rows, int split_k, pia_gemm_plan_t **out) {
+  PIA_REQUIRE(d_w && d_scale && d_x && out, "null argument");
+  PIA_REQUIRE(groups >= 1 && groups <= 65535, "groups %d outside [1, 65535]", groups);
+  PIA_REQUIRE(N > 0 && K > 0 && N % BMW == 0 && K % F8_BK == 0, "fp8 weights need N %% %d == 0 and K %% %d == 0 (N = %d, K = %d)",
+              BMW, F8_BK, N, K);
+  PIA_REQUIRE(x_rows >= 1 && x_rows <= 256, "the activation buffer of an fp8 plan holds 1..256 rows, not %d", x_rows);
+  PIA_REQUIRE((reinterpret_cast<uintptr_t>(d_w) & 15) == 0 && (reinterpret_cast<uintptr_t>(d_x) & 15) == 0 &&
+              (reinterpret_cast<uintptr_t>(d_scale) & 3) == 0 && (reinterpret_cast<uintptr_t>(d_bias) & 1) == 0,
+              "operands must be aligned (weights / activations 16 bytes)");
+  const int n_chunks = K / F8_BK;
+  const int want_cluster = (split_k == -2 || split_k == -4 || split_k == -8) ? -split_k : 0;
+  PIA_REQUIRE(split_k >= 1 || want_cluster, "fp8 plans take split_k >= 1 or a cluster split of -2, -4 or -8");
+  PIA_REQUIRE(groups == 1 || split_k == 1, "grouped fp8 plans do not split K");
+  if (want_cluster) split_k = want_cluster;
+  if (split_k > n_chunks) split_k = n_chunks;
+  pia_gemm_plan *g = new (std::nothrow) pia_gemm_plan();
+  PIA_REQUIRE(g, "out of host memory");
+  g->fp8 = 1;
+  g->tok = x_rows <= 64 ? 64 : x_rows <= 128 ? 128 : 256;
+  g->x_rows = x_rows;
+  Params &p = g->p;
+  p.N = N; p.K = K; p.n_chunks = n_chunks;
+  p.chunks_per_split = (n_chunks + split_k - 1) / split_k;
+  p.n_split = (n_chunks + p.chunks_per_split - 1) / p.chunks_per_split;
+  p.rows = g->tok; p.out_bf16 = nullptr; p.out_f32 = nullptr; p.silu = 0; p.tiled = 1; p.cluster = 0;
+  p.groups = groups; p.w_group_rows = N; p.x_group_chunks = K / BK; p.out_group_stride = (long long)g->tok * N;
+  p.scale = d_scale; p.bias = (const __nv_bfloat16 *)d_bias; p.w_group_tiles = N / BMW;
+  g->stream_k = 0; g->no_pdl = 0;
+  if (want_cluster) {
+    if (p.n_split != want_cluster) { delete g; set_error("K = %d is too short for %d cluster splits", K, want_cluster); return PIA_ERR_INVALID; }
+    p.cluster = want_cluster;
+  }
+  int rc = encode_tiled_w_fp8(&g->map_w, d_w, (uint64_t)groups * (N / BMW) * n_chunks);
+  if (rc == PIA_OK) rc = encode_2d(&g->map_x, d_x, (uint64_t)groups * K, (uint64_t)x_rows, BK, g->tok, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
+  if (rc == PIA_OK) {
+    int n_sm = 148, dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
+    const int ctas = (N / BMW) * p.n_split * groups;
+    g->nstage = g->tok == 64 ? (ctas <= n_sm ? 5 : 2) : g->tok == 128 ? 4 : 2;
+    cudaError_t e = g->tok == 64 ? (g->nstage == 5 ? f8_attr<5, 64>() : f8_attr<2, 64>())
+                  : g->tok == 128 ? f8_attr<4, 128>() : f8_attr<2, 256>();
+    if (e != cudaSuccess) { set_error("cudaFuncSetAttribute: %s", cudaGetErrorString(e)); rc = PIA_ERR_CUDA; }
+  }
+  if (rc != PIA_OK) { delete g; return rc; }
+  *out = g;
+  return PIA_OK;
+}
+
+extern "C" int pia_gemm_plan_create_fp8(const void *d_w_tiled_f8, const float *d_scale, const void *d_bias, int N, int K,
+                                        const void *d_x, int x_rows, int split_k, pia_gemm_plan_t **out) {
+  return fp8_plan_create(d_w_tiled_f8, d_scale, d_bias, 1, N, K, d_x, x_rows, split_k, out);
+}
+
+extern "C" int pia_gemm_plan_create_grouped_fp8(const void *d_w_tiled_f8, const float *d_scale, int groups, int N, int K,
+                                                const void *d_x, int x_rows, pia_gemm_plan_t **out) {
+  return fp8_plan_create(d_w_tiled_f8, d_scale, nullptr, groups, N, K, d_x, x_rows, 1, out);
+}
+
 struct PdlScope { int on; explicit PdlScope(int off) : on(off) { if (on) ++pia::g_pdl_off; } ~PdlScope() { if (on) --pia::g_pdl_off; } };
 
 extern "C" int pia_gemm_run(pia_gemm_plan_t *g, int rows, void *d_out, void *stream) {
   PIA_REQUIRE(g && d_out, "null argument");
+  if (g->fp8) {
+    PIA_REQUIRE(rows >= 1 && rows <= g->x_rows, "rows %d outside [1,%d]", rows, g->x_rows);
+    PdlScope pdl_scope(g->no_pdl);
+    Params p = g->p;
+    p.rows = rows; p.no_pdl = g->no_pdl;
+    if (p.n_split == 1 || p.cluster) p.out_bf16 = (__nv_bfloat16 *)d_out; else p.out_f32 = (float *)d_out;
+    cudaStream_t st = (cudaStream_t)stream;
+    const cudaError_t e = g->tok == 64 ? (g->nstage == 5 ? f8_launch<5, 64>(g, p, st) : f8_launch<2, 64>(g, p, st))
+                        : g->tok == 128 ? f8_launch<4, 128>(g, p, st) : f8_launch<2, 256>(g, p, st);
+    PIA_CUDA_CHECK(e);
+    count_launch();
+    return PIA_OK;
+  }
   PIA_REQUIRE(rows >= 1 && rows <= TOK, "rows %d outside [1,%d]", rows, TOK);
   PdlScope pdl_scope(g->no_pdl);
   if (g->stream_k) {

@@ -109,6 +109,10 @@ class GPT2LMHeadModel(LookaheadPreTrainedModel):
                 torch.zeros((max_pos, PAD_D // 2), dtype=torch.bfloat16, device=dev))
 
     @torch.no_grad()
+    def quantize_weights(self, dtype=None):
+        raise ValueError('fp8 weights are not built for GPT-2: its Conv1D projections run through torch, not the '
+                         'weight-streaming GEMM')
+
     def fuse(self):
         """c_attn / c_proj re-laid out for 128-wide (zero padded) heads; done once, outside any captured graph"""
         if self._fused:

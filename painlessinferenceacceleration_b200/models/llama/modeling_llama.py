@@ -100,10 +100,14 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         return self
 
     @classmethod
-    def from_pretrained(cls, path, torch_dtype=torch.bfloat16, device=None, **kwargs):
-        """HF checkpoint directory (config.json + *.safetensors / pytorch_model*.bin) -> model on the GPU"""
+    def from_pretrained(cls, path, torch_dtype=torch.bfloat16, device=None, weight_dtype=None, **kwargs):
+        """HF checkpoint directory (config.json + *.safetensors / pytorch_model*.bin) -> model on the GPU.
+        weight_dtype=torch.float8_e4m3fn: load the bf16 checkpoint, then quantize_weights() (fp8 projections)"""
         from transformers import AutoConfig
         config = AutoConfig.from_pretrained(path)
+        _reject_prequantised(config)
+        if weight_dtype not in (None, torch_dtype, torch.float8_e4m3fn):
+            raise ValueError(f'weight_dtype {weight_dtype} is not built (bf16 or torch.float8_e4m3fn)')
         model = cls(config, device=device, dtype=torch_dtype)
         files = sorted(glob.glob(os.path.join(path, '*.safetensors')))
         own = dict(model.named_parameters())
@@ -126,6 +130,8 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         missing = [k for k in own if k not in seen]
         if missing:
             raise RuntimeError(f'checkpoint is missing {len(missing)} tensors, e.g. {missing[:4]}')
+        if weight_dtype == torch.float8_e4m3fn:
+            model.quantize_weights(weight_dtype)
         return model
 
     def _convert_checkpoint_keys(self, sd):
@@ -157,6 +163,71 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         ni = m.gate_proj.weight.shape[0]
         m.gate_proj.weight.data, m.up_proj.weight.data = w[:ni], w[ni:]
         m.gate_up_weight = w
+
+    # ------------------------------------------------------------------ fp8 weight-only quantisation
+    @property
+    def quantized(self):
+        return self.__dict__.get('_fp8', False)
+
+    def _fp8_targets(self, layer):
+        """(module, name, [N, K]) of the projections quantize_weights() replaces in one layer (after fuse())"""
+        c = self.config
+        hd = self.geometry()['head_dim']
+        kv = getattr(c, 'num_key_value_heads', None) or c.num_attention_heads
+        H, nq = c.hidden_size, c.num_attention_heads * hd
+        a, m = layer.self_attn, layer.mlp
+        return [(a, 'qkv', (nq + 2 * kv * hd, H)), (a, 'o', (H, nq)),
+                (m, 'gate_up', (2 * c.intermediate_size, H)), (m, 'down', (H, c.intermediate_size))]
+
+    @torch.no_grad()
+    def quantize_weights(self, dtype=torch.float8_e4m3fn):
+        """Weight-only FP8: every decoder projection (fused qkv, o, fused gate/up, down; Mixtral's stacked experts)
+        becomes e4m3 tiles plus one fp32 scale per output channel (ops.quantize_fp8, include/pia_b200.h) and from then
+        on runs on the fp8 GEMM plans; the embedding, the norms, the MoE router and lm_head stay bf16.  Layer by layer,
+        so that peak memory is the model plus one layer's bf16 projections; the bf16 storage is freed (the HF-named
+        q/k/v/o/gate/up/down parameters are removed).  Irreversible; lookahead decoding stays lossless with respect to
+        the quantised model."""
+        if dtype != torch.float8_e4m3fn:
+            raise ValueError(f'quantize_weights: {dtype} is not built (torch.float8_e4m3fn)')
+        if self.quantized:
+            return self
+        _reject_prequantised(self.config)
+        for mod, name, (N, K) in self._fp8_targets(self.model.layers[0]):
+            if N % 128 or K % 128:
+                raise ValueError(f'quantize_weights: the {name} projection is [{N}, {K}]; fp8 weights need both '
+                                 'dimensions to be multiples of 128')
+        self.fuse()
+        self._rt = None                              # its GEMM plans hold the bf16 operands
+        self.__dict__.pop('_tiled_weights', None)
+        for layer in self.model.layers:
+            self._quantize_layer(layer)
+        self._fp8 = True
+        if torch.cuda.is_available() and self.device.type == 'cuda':
+            torch.cuda.empty_cache()
+        return self
+
+    @staticmethod
+    def _put_fp8(mod, name, w):
+        wq, s = ops.quantize_fp8(w)
+        mod.register_buffer(name + '_fp8', ops.tile_weight_fp8(wq))
+        mod.register_buffer(name + '_scale', s.contiguous())
+
+    def _quantize_layer(self, layer):
+        a = layer.self_attn
+        self._put_fp8(a, 'qkv', a.qkv_weight)
+        self._put_fp8(a, 'o', a.o_proj.weight)
+        bias = a.qkv_bias
+        del a.q_proj, a.k_proj, a.v_proj, a.o_proj, a.qkv_bias
+        a.qkv_weight = None
+        a.register_buffer('qkv_bias', bias)     # None for Llama / Mistral / Mixtral
+        self._quantize_mlp(layer)
+
+    def _quantize_mlp(self, layer):
+        m = layer.mlp
+        self._put_fp8(m, 'gate_up', m.gate_up_weight)
+        self._put_fp8(m, 'down', m.down_proj.weight)
+        del m.gate_proj, m.up_proj, m.down_proj
+        m.gate_up_weight = None
 
     # ------------------------------------------------------------------ geometry / tables
     def geometry(self):
@@ -199,6 +270,8 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         plans = getattr(rt, 'gemm_plans', None)
         if plans is not None:
             return plans
+        if self.quantized:
+            return self._fp8_gemm_plans(rt)
         import os
         if os.environ.get('PIA_GEMM', '1') == '0' or rt.max_nodes != 64:
             rt.gemm_plans = False
@@ -252,6 +325,53 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
                 plans[name].set_pdl(False)
         return plans
 
+    # split-K of the narrow fp8 projections (1: none, 4: fp32 slices summed by the next rmsnorm, -2 / -4: 2 / 4 K
+    # splits as one cluster reducing through DSMEM).  Chosen in the whole verify forward (64 rows, one CUDA graph) at
+    # the Llama-2-7B shape, one choice changed at a time (scripts/bench_fp8.py, B200 at 1000 W / 1965 MHz, us):
+    #   qkv -2, o -4, down -4: 4285 | qkv 1: 4414, qkv -4: 4385 | o 1: 4831, o 4: 4305, o -2: 4459 |
+    #   down 1: 5951, down 4: 4325, down -2: 4863
+    FP8_SPLIT = dict(qkv=-2, o=-4, down=-4)
+
+    def _fp8_gemm_plans(self, rt):
+        """every projection of a quantised model on fp8 plans: the decode buffers (64 or 128 rows) and the 256-row
+        prefill buffers; lm_head stays bf16 (k_gemm_ws plan at 64 rows, as for bf16 models)"""
+        g = rt.g
+        plans = {}
+        for b in (rt.decode_bufs, rt.prefill_bufs):
+            dev = b.y.device
+            b.gu = torch.zeros((b.rows, 2 * g['inter']), dtype=torch.bfloat16, device=dev)
+            b.act = torch.zeros((b.rows, g['inter']), dtype=torch.bfloat16, device=dev)
+            b.fp8_plans = {'layers': [self._fp8_layer_plans(layer, b) for layer in self.model.layers]}
+        plans = rt.decode_bufs.fp8_plans
+        if rt.max_nodes == 64:
+            plans['lm_head'] = self._mk_gemm(self.lm_head.weight.data, rt.decode_bufs.y)
+        rt.gemm_plans = plans
+        return plans
+
+    @staticmethod
+    def _fp8_split(split_k, w):
+        """the configured split for a tiled fp8 weight, halved while its K (in 128-wide chunks) cannot give every CTA of
+        a cluster split a share (small models)"""
+        chunks = w.shape[-3]
+        c = -split_k
+        while c > 1 and -(-chunks // -(-chunks // c)) != c:
+            c //= 2
+        return split_k if split_k >= 1 else (-c if c > 1 else 1)
+
+    def _fp8_layer_plans(self, layer, b):
+        a, sk = layer.self_attn, self.FP8_SPLIT
+        plans = {'qkv': ops.Gemm.fp8(a.qkv_fp8, a.qkv_scale, b.y, bias=a.qkv_bias,
+                                     split_k=self._fp8_split(sk['qkv'], a.qkv_fp8)),
+                 'o': ops.Gemm.fp8(a.o_fp8, a.o_scale, b.attn, split_k=self._fp8_split(sk['o'], a.o_fp8))}
+        plans.update(self._fp8_mlp_plans(layer, b))
+        return plans
+
+    def _fp8_mlp_plans(self, layer, b):
+        m = layer.mlp
+        return {'gate_up': ops.Gemm.fp8(m.gate_up_fp8, m.gate_up_scale, b.y),
+                'down': ops.Gemm.fp8(m.down_fp8, m.down_scale, b.act,
+                                     split_k=self._fp8_split(self.FP8_SPLIT['down'], m.down_fp8))}
+
     def _mk_gemm(self, w, x, split_k=1):
         """HBM-tiled copy of the weight when its row count allows it (N % 128 == 0), else the row-major tensor.
         The tiled copies belong to the model (one per weight), not to a runtime: rebuilding the runtime for a longer
@@ -301,23 +421,23 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         pf['dirty'] = True
 
     # ------------------------------------------------------------------ the verify forward on static buffers
-    def _mlp(self, rt, layer, y, plans=None, pf=None):
+    def _mlp(self, rt, layer, y, plans=None, pf=None, b=None):
         """returns (x, parts): the MLP output as a bf16 tensor or as fp32 split-K slices for the next rmsnorm"""
         m = layer.mlp
         if plans:
-            b = rt.decode_bufs
+            b = b if b is not None else rt.decode_bufs
             if 'gate_up_silu' in plans:
-                plans['gate_up_silu'].run(64, out=b.act)
+                plans['gate_up_silu'].run(b.rows, out=b.act)
             else:
                 if 'gate_up' in plans:
-                    plans['gate_up'].run(64, out=b.gu)
+                    plans['gate_up'].run(b.rows, out=b.gu)
                 else:
                     torch.mm(y, m.gate_up_weight.t(), out=b.gu)
                 if pf:
                     self._prefetch(pf, [(m.down_proj.weight, pf['down'], 0)])
                 ops.silu_mul(b.gu, b.act)
             if 'down' in plans:
-                o = plans['down'].run(64)
+                o = plans['down'].run(b.rows)
                 return (o, None) if plans['down'].splits == 1 else (None, o)
             return torch.mm(b.act, m.down_proj.weight.t()), None
         gu = torch.mm(y, m.gate_up_weight.t())
@@ -336,8 +456,12 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
         g = rt.g
         eps = self.config.rms_norm_eps
         ops.embed_gather(self.model.embed_tokens.weight, b.ids, b.n_total, b.h)
-        plans = self._gemm_plans(rt) if b is rt.decode_bufs else False
-        pf = self._prefetch_cfg(rt) if plans else False
+        if self.quantized:   # every projection on fp8 plans, prefill passes included
+            plans = self._gemm_plans(rt) if b is rt.decode_bufs else b.fp8_plans
+            pf = False
+        else:
+            plans = self._gemm_plans(rt) if b is rt.decode_bufs else False
+            pf = self._prefetch_cfg(rt) if plans else False
         fused_attn = b is rt.decode_bufs and os.environ.get('PIA_ATTN_FUSED', '0') != '0' and \
             (b.slots.batch == 1 or b.slots.kv_slot_stride != 0)
         x, parts, resid_in = b.h, None, None  # norm(x | parts, resid_in) -> (resid = x + resid_in, y = norm(resid))
@@ -353,7 +477,7 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
             norm(layer.input_layernorm.weight)
             a = layer.self_attn
             if lp and 'qkv' in lp:
-                lp['qkv'].run(64, out=b.qkv)
+                lp['qkv'].run(b.rows, out=b.qkv)
             elif a.qkv_bias is not None:   # Qwen2: cuBLASLt bias epilogue, one rounding of the fp32 xW^T + b
                 torch.addmm(a.qkv_bias, b.y, a.qkv_weight.t(), out=b.qkv)
             else:
@@ -370,22 +494,30 @@ class LlamaForCausalLM(LookaheadPreTrainedModel):
                                    rt.rope_sin, b.q, rt.k_layer(li, b.kv_slot), rt.v_layer(li, b.kv_slot), rt.max_seq)
                 rt.plan.forward(li, b.q, b.mask, b.slots, b.attn)
             if lp and 'o' in lp:
-                o = lp['o'].run(64)
+                o = lp['o'].run(b.rows)
                 x, parts, resid_in = (o, None, b.resid) if lp['o'].splits == 1 else (None, o, b.resid)
             else:
                 x, parts, resid_in = torch.mm(b.attn, a.o_proj.weight.t()), None, b.resid
             norm(layer.post_attention_layernorm.weight)
-            x, parts = self._mlp(rt, layer, b.y, lp, pf)
+            x, parts = self._mlp(rt, layer, b.y, lp, pf, b)
         if pf and pf.pop('dirty', False):  # join the side stream (required before a capture ends)
             torch.cuda.current_stream().wait_stream(pf['side'])
         if last_only:
             return
         norm(self.model.norm.weight)
         if b.logits is not None:
-            if plans:
-                plans['lm_head'].run(64, out=b.logits)
+            if plans and 'lm_head' in plans:
+                plans['lm_head'].run(b.rows, out=b.logits)
             else:
                 torch.mm(b.y, self.lm_head.weight.t(), out=b.logits)
+
+
+def _reject_prequantised(config):
+    q = getattr(config, 'quantization_config', None)
+    if q:
+        method = q.get('quant_method', '?') if isinstance(q, dict) else getattr(q, 'quant_method', '?')
+        raise ValueError(f'pre-quantised checkpoints ({method}) are not built: load the bf16 checkpoint with '
+                         'weight_dtype=torch.float8_e4m3fn to serve fp8 weights')
 
 
 class LlamaPreTrainedModel(LookaheadPreTrainedModel):

@@ -102,25 +102,49 @@ class MixtralForCausalLM(LlamaForCausalLM):
         inter = two_i // 2
         if os.environ.get('PIA_MOE_GEMM', '1') == '0' or H % 128 or H % 64 or inter % 64 or (E * two_i) % 128:
             return {}
-        dev = b.y.device
-        if not hasattr(b, 'moe_gu'):
-            b.moe_gu = torch.zeros((b.rows, E * two_i), dtype=torch.bfloat16, device=dev)
-            b.moe_act = torch.zeros((b.rows, E * inter), dtype=torch.bfloat16, device=dev)
-            b.moe_out = torch.zeros((b.rows, H), dtype=torch.bfloat16, device=dev)
-            b.moe_dense = torch.zeros((b.rows, E), dtype=torch.bfloat16, device=dev)
+        self._moe_bufs(b, E, inter, H)
         return {'moe_gate_up': ops.Gemm(moe.experts.gate_up_proj.data.view(E * two_i, H), b.y),
                 'moe_down': ops.Gemm.grouped(moe.experts.down_proj.data, b.moe_act)}
 
-    def _mlp(self, rt, layer, y, plans=None, pf=None):
+    @staticmethod
+    def _moe_bufs(b, E, inter, H):
+        if not hasattr(b, 'moe_gu'):
+            dev = b.y.device
+            b.moe_gu = torch.zeros((b.rows, E * 2 * inter), dtype=torch.bfloat16, device=dev)
+            b.moe_act = torch.zeros((b.rows, E * inter), dtype=torch.bfloat16, device=dev)
+            b.moe_out = torch.zeros((b.rows, H), dtype=torch.bfloat16, device=dev)
+            b.moe_dense = torch.zeros((b.rows, E), dtype=torch.bfloat16, device=dev)
+
+    def _quantize_mlp(self, layer):
+        """stacked experts: gate_up [E, 2I, H] -> one fp8 weight [E*2I, H] (one plan over all experts, as the bf16
+        path), down [E, H, I] -> per-expert tiles + scales [E, H] for the grouped plan"""
+        ex = layer.mlp.experts
+        E, two_i, H = ex.gate_up_proj.shape
+        wq, s = ops.quantize_fp8(ex.gate_up_proj.data)
+        ex.register_buffer('gate_up_fp8', ops.tile_weight_fp8(wq.view(E * two_i, H)))
+        ex.register_buffer('gate_up_scale', s.reshape(E * two_i).contiguous())
+        del wq
+        wq, s = ops.quantize_fp8(ex.down_proj.data)
+        ex.register_buffer('down_fp8', ops.tile_weight_fp8(wq))
+        ex.register_buffer('down_scale', s.contiguous())
+        del ex.gate_up_proj, ex.down_proj
+
+    def _fp8_mlp_plans(self, layer, b):
+        moe, c = layer.mlp, self.config
+        self._moe_bufs(b, moe.num_experts, c.intermediate_size, c.hidden_size)
+        return {'moe_gate_up': ops.Gemm.fp8(moe.experts.gate_up_fp8, moe.experts.gate_up_scale, b.y),
+                'moe_down': ops.Gemm.grouped_fp8(moe.experts.down_fp8, moe.experts.down_scale, b.moe_act)}
+
+    def _mlp(self, rt, layer, y, plans=None, pf=None, b=None):
         moe = layer.mlp
         if plans:
-            b = rt.decode_bufs
+            b = b if b is not None else rt.decode_bufs
             E = moe.num_experts
-            inter = moe.experts.down_proj.shape[2]
+            inter = self.config.intermediate_size
             ops.moe_router(y, moe.gate.weight, moe.top_k, b.moe_dense)              # :721-727 in one kernel
-            plans['moe_gate_up'].run(64, out=b.moe_gu)
+            plans['moe_gate_up'].run(b.rows, out=b.moe_gu)
             ops.silu_mul(b.moe_gu.view(b.rows * E, 2 * inter), b.moe_act.view(b.rows * E, inter))
-            ye = plans['moe_down'].run(64)                                          # [E, 64, H]
+            ye = plans['moe_down'].run(b.rows)                                      # [E, rows, H]
             ops.moe_combine(ye, b.moe_dense, b.moe_out)
             return b.moe_out, None
         dense = torch.empty((y.shape[0], moe.num_experts), dtype=y.dtype, device=y.device)
